@@ -8,6 +8,7 @@ q,k,v at the HunyuanVideo 720x1280x125f shape: q,k,v [1, 115456, 24, 128] bf16
 p_remain 0.3, text_amp 0, 26-neighbour adjacency of the 32x45x80 gilbert curve).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--drop 0.7]
+                    [--dump-outputs DIR]
 
 N>1 (torchrun): Ulysses — image tokens sharded over ranks outside the operator, all-to-all to
 (all tokens x H/N heads) inside (jenga_b200.ulysses), strong scaling of the same layer.
@@ -22,6 +23,9 @@ roofline         attention kernel alone (CUDA events on its stream), vs the meas
 cpu_baseline     the oracle port (oracle/attention_oracle.py) on the host cores, bounded sample.
 --impl reference the reference's CPU-runnable path for this operator (torch SDPA with the
                  expanded block mask, hyvideo/modules/attenion.py:102-107) on a bounded sample.
+--dump-outputs   writes the operator output of the last timed step as DIR/out.npy (float32; under
+                 N>1 each rank's token slice as DIR/out_rank<r>.npy).  Inputs are seeded, so two
+                 builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -488,6 +492,24 @@ def dit_forward_leg(wl, inp, n_double, n_single, hidden=3072, heads=24, fp8_too=
         return {"unavailable": f"{type(e).__name__}: {str(e)[:300]}", "trace": traceback.format_exc()[-600:]}
 
 
+DUMP_LIMIT_BYTES = 48_000_000   # what all dumped files may add up to, with room for .npy headers
+
+
+def dump_output(out: torch.Tensor, path: Path, limit: int = DUMP_LIMIT_BYTES) -> None:
+    """Writes `out` ([1, rows, ...], one row per token) as float32 .npy.  An output over `limit`
+    bytes is reduced to a fixed sample of whole rows (seeded, sorted, the same for every run of
+    the same shape)."""
+    import numpy as np
+    x = out.detach().reshape(out.shape[1], -1)
+    rows, cols = x.shape
+    keep = max(1, min(rows, limit // (4 * cols)))
+    if keep < rows:
+        idx = torch.randperm(rows, generator=torch.Generator().manual_seed(0))[:keep].sort().values
+        x = x[idx.to(x.device)]
+    path.parent.mkdir(parents=True, exist_ok=True)
+    np.save(path, x.float().cpu().numpy())
+
+
 # ------------------------------------------------------------------------------------------------
 def main():
     ap = argparse.ArgumentParser()
@@ -510,7 +532,14 @@ def main():
                     help="ALSO time the opt-in FP8 P.V variant (reported under 'fp8_pv_variant'; never the headline)")
     ap.add_argument("--no-gpu-reference", action="store_true",
                     help="skip timing the unmodified reference operator (Triton + FA2) on this GPU")
+    ap.add_argument("--dump-outputs", metavar="DIR", type=Path,
+                    help="write the operator output of the last timed step to DIR/out.npy (float32; a "
+                         "fixed sample of its rows when it exceeds 48 MB)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     wl = workload(args.workload, args.drop)
     rank = int(os.environ.get("RANK", "0"))
@@ -581,10 +610,15 @@ def main():
     with ClockSampler(local_rank) as clk:
         ev0.record()
         for _ in range(args.steps):
-            step()
+            last = step()
         ev1.record()
         barrier()
     ms = ev0.elapsed_time(ev1) / args.steps
+    if args.dump_outputs:
+        # rows: under N>1 this rank's share of the budget, so that the ranks' files stay within it
+        dump_output(last, args.dump_outputs / ("out.npy" if world == 1 else f"out_rank{rank}.npy"),
+                    DUMP_LIMIT_BYTES // world)
+    del last
     if dist is not None:
         t = torch.tensor([ms], device=dev)
         dist.all_reduce(t, op=dist.ReduceOp.MAX)

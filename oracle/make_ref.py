@@ -17,6 +17,7 @@ from __future__ import annotations
 
 import hashlib
 import json
+import os
 import shutil
 import sys
 from pathlib import Path
@@ -58,10 +59,19 @@ FILES = [
 ]
 
 
+def readable_dir(p: Path) -> bool:
+    """True iff `p` is a directory this process may read (a directory behind one it may not
+    enter counts as absent instead of raising PermissionError)."""
+    try:
+        return p.is_dir() and os.access(p, os.R_OK | os.X_OK)
+    except OSError:
+        return False
+
+
 def materialise(src: Path = SRC, dst: Path = DST, quiet: bool = False) -> Path | None:
     """Copies FILES from `src` to `dst`.  Returns dst, or None when the reference is not mounted
     and nothing was materialised earlier (callers skip reference-backed checks then)."""
-    if not src.is_dir():
+    if not readable_dir(src):
         return dst if (dst / "MANIFEST.json").exists() else None
     manifest = {}
     for rel in FILES:

@@ -35,11 +35,11 @@ def ref_root() -> Path | None:
     """The directory holding the unmodified reference files, or None."""
     import os
     live = Path("/root/reference")
-    if (live / "gilbert.py").is_file() and os.environ.get("JENGA_ORACLE_REF") != "staged":
+    from . import make_ref
+    if make_ref.readable_dir(live) and (live / "gilbert.py").is_file() and os.environ.get("JENGA_ORACLE_REF") != "staged":
         return live
     staged = HERE / "_ref"
     if (staged / "MANIFEST.json").is_file():
-        from . import make_ref
         if not make_ref.verify(staged):
             raise RuntimeError("oracle/_ref/ does not match its manifest: the reference copy was modified")
         return staged

@@ -197,13 +197,15 @@ def test_unmodified_wan_self_attention_through_install_hook(modules):
     _compare(ra, oa, row_ok, "WanSelfAttention")
 
 
-def test_token_reorder_is_routed_to_the_gather_kernel(modules):
-    """jenga_hyvideo.py:116-118,226: img[:, hilbert_order], freqs[hilbert_order], img[:, linear_to_hilbert]."""
+def test_token_reorder_is_routed_to_the_gather_kernel():
+    """jenga_hyvideo.py:116-118,226: img[:, hilbert_order], freqs[hilbert_order], img[:, linear_to_hilbert].
+    Needs no reference file: the hook sees plain tensor indexing."""
     from jenga_b200 import blocks, gilbert
     l2h, h2l = gilbert.mapping_tensors(8, 16, 16)
     l2h, h2l = l2h.cuda(), h2l.cuda()
     img = torch.randn(1, 2048, 512, device="cuda").bfloat16()
     cos = torch.randn(2048, 128, device="cuda")
+    was_installed = blocks._gather_mode is not None
     blocks.install_gather_hook()
     before = blocks.STATS["gather"]
     a = img[:, h2l]
@@ -211,5 +213,8 @@ def test_token_reorder_is_routed_to_the_gather_kernel(modules):
     back = a[:, l2h]
     assert blocks.STATS["gather"] == before + 3
     blocks.remove_gather_hook()
-    assert torch.equal(a, img[:, h2l]) and torch.equal(b, cos[h2l]) and torch.equal(back, img)
-    blocks.install_gather_hook()
+    try:
+        assert torch.equal(a, img[:, h2l]) and torch.equal(b, cos[h2l]) and torch.equal(back, img)
+    finally:
+        if was_installed:
+            blocks.install_gather_hook()
